@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path (through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host CPUs
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 Metric (BASELINE.json): Gpoint/s (complex) for a 2^20-point f64 forward FFT, planar re/im.
 A "step" is one in-place forward FFT of one 2^20-point signal through
@@ -358,6 +359,31 @@ def timed(c, step, K, graph=None, group=1, graph_rem=None):
     return ms_total / K, launched
 
 
+DUMP_MAX_ELEMS = 1 << 21                  # per dumped array: at most 16 MiB of f64 / 8 MiB of f32
+DUMP_MAX_BYTES = 64 * 1024 * 1024
+
+
+def dump_sample(t, seed=1234):
+    """A 1-D device tensor as a host array: whole up to DUMP_MAX_ELEMS elements, else a fixed seeded sample of its
+    elements in index order (the same indices in every run of the same workload)."""
+    import torch
+    if t.numel() <= DUMP_MAX_ELEMS:
+        return t.cpu().numpy()
+    idx = np.sort(np.random.default_rng(seed).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+    return t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+
+
+def write_dump(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, total
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(d / f"{name}.npy", a)
+    print(f"[bench] dumped {sorted(arrays)} ({total / 2**20:.1f} MiB) to {d}", file=sys.stderr, flush=True)
+
+
 def per_pass_times(c, sfx, planner, get, batch, n, reps):
     fprof = c.lib.fn("phastft_fft_dit_{s}_dev_profile", sfx)
     pass_ms = (C.c_float * 3)()
@@ -372,7 +398,9 @@ def per_pass_times(c, sfx, planner, get, batch, n, reps):
 
 
 # ---- C4: 4096 x 2^16 f32, sharded over the ranks (strong scaling), the reference's caller loop examples/benchmark.rs:24-36 ----
-def measure_batch(c, K, W, with_e2e=True):
+def measure_batch(c, K, W, with_e2e=True, dump=None):
+    """`dump`: a dict that receives, as batch_f32_re / batch_f32_im [transforms, 2^16], a fixed seeded sample of the
+    transforms the last timed step computes from the seeded inputs."""
     torch, pf, _lib = c.torch, c.pf, c.lib
     n, total = 1 << 16, 4096
     lo, hi = c.shard_range(total, c.rank, c.world)
@@ -388,6 +416,8 @@ def measure_batch(c, K, W, with_e2e=True):
     full_re = torch.rand(total * n, dtype=torch.float32, device=c.dev, generator=g) * 2 - 1
     full_im = torch.rand(total * n, dtype=torch.float32, device=c.dev, generator=g) * 2 - 1
     re = full_re[lo * n:hi * n].clone(); im = full_im[lo * n:hi * n].clone()
+    # every step transforms the shard in place, so after a few steps it holds inf / NaN; the dumped step starts again from a copy
+    seeded = (re.clone(), im.clone()) if dump is not None else None
     f = _lib.fn("phastft_fft_dit_{s}_dev", "f32")
 
     def step(i):
@@ -426,6 +456,15 @@ def measure_batch(c, K, W, with_e2e=True):
         step(i)
     torch.cuda.synchronize()
     ms_per_step, launched = timed(c, step, K)
+    if seeded is not None:
+        re.copy_(seeded[0]); im.copy_(seeded[1])
+        del seeded
+        step(K - 1)
+        torch.cuda.synchronize()
+        picks = np.sort(np.random.default_rng(1234).choice(nb, min(nb, DUMP_MAX_ELEMS // n), replace=False))
+        rows = torch.from_numpy(picks).to(c.dev)
+        dump["batch_f32_re"] = re.view(nb, n)[rows].cpu().numpy()
+        dump["batch_f32_im"] = im.view(nb, n)[rows].cpu().numpy()
     value = total * n / (ms_per_step * 1e-3) / 1e9
     alone = per_pass_times(c, "f32", planner, lambda b: (re, im), nb, n, 5)
     alg = 2 * n * 4 * 2 * nb                   # this rank's shard; the fraction is per GPU (every rank streams its own HBM)
@@ -467,10 +506,13 @@ def run_ours(args):
     sampler.start()
     extra = {}
     roofline = e2e = None
+    dump = {} if args.dump_outputs else None
 
     if wl == "batch_f32":
-        out, planner = measure_batch(c, K, W, with_e2e=True)
+        out, planner = measure_batch(c, K, W, with_e2e=True, dump=dump)
         clocks = sampler.stop()
+        if rank == 0 and dump is not None:
+            write_dump(args.dump_outputs, dump)
         cpu = None
         if rank == 0 and world == 1 and not args.no_cpu_baseline:
             _, _, cpu = cpu_reference_run(wl, steps=30, warmup=2, budget_s=25.0)
@@ -556,9 +598,25 @@ def run_ours(args):
             step(0)
         torch.cuda.synchronize()
     reset()
+    seeded = None
+    if dump is not None and wl != "r2c_f64_2p24":
+        # the c2c steps transform their buffers in place, so after ~100 passes over a buffer it holds inf / NaN: keep the last
+        # step's seeded input and run that step once more from it after the timed loop
+        last = (K - 1) % nbuf
+        seeded = (bufs_re[last].clone(), bufs_im[last].clone())
     ms_per_step, launches = timed(c, step, K, graph, group, graph_rem)
     if graph is not None:
         launches += K * planner_passes(planner)          # graph replays launch kernels without entering the library
+    if dump is not None:
+        if seeded is not None:
+            bufs_re[last].copy_(seeded[0]); bufs_im[last].copy_(seeded[1])
+            del seeded
+            step(K - 1)
+            torch.cuda.synchronize()
+            dump["c2c_re"], dump["c2c_im"] = dump_sample(bufs_re[last]), dump_sample(bufs_im[last])
+        else:
+            torch.cuda.synchronize()
+            dump["r2c_re"], dump["r2c_im"], dump["c2r_out"] = dump_sample(sre), dump_sample(sim), dump_sample(y)
     value = world * points_per_step / (ms_per_step * 1e-3) / 1e9
 
     # ---- roofline: whole-transform fraction from the timed region; per-pass split from CUDA events, live, on the launching stream ----
@@ -622,8 +680,10 @@ def run_ours(args):
     if wl == "c2c_f64_2p20" and not args.no_batched:
         del bufs_re, bufs_im
         torch.cuda.empty_cache()
-        batched, _ = measure_batch(c, 20, 3, with_e2e=True)
+        batched, _ = measure_batch(c, min(K, 20), 3, with_e2e=True, dump=dump)      # --steps also bounds this leg
     clocks = sampler.stop()
+    if rank == 0 and dump is not None:
+        write_dump(args.dump_outputs, dump)
 
     # ---- CPU baseline beside it (rank 0, N = 1 only; bounded sample) ------------------------------------
     cpu = None
@@ -655,7 +715,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="issue every step through the C ABI instead of replaying a captured CUDA graph")
     ap.add_argument("--no-batched", action="store_true", help="skip the 4096 x 2^16 f32 sharded measurement that the default workload adds as `batched`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computes from its seeded inputs as DIR/<name>.npy "
+                         "(f32 / f64, at most 64 MiB in all; arrays longer than 2^21 as a fixed seeded sample): c2c_re / c2c_im, "
+                         "batch_f32_re / batch_f32_im (a seeded sample of [transforms, 2^16]), r2c_re / r2c_im / c2r_out.  The inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     # defaults sized so the timed region lasts ~0.2-0.5 s (clock sampling needs that) and a run takes < 2 min
     dflt = {"c2c_f64_2p20": (20000, 200), "c2c_f64_2p26": (100, 5), "batch_f32": (100, 5), "r2c_f64_2p24": (200, 10)}[args.workload]
     if args.impl == "reference":
@@ -664,6 +731,8 @@ def main():
         args.steps = dflt[0]
     if args.warmup is None:
         args.warmup = dflt[1]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

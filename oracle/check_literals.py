@@ -2,11 +2,13 @@
 """Verify that the oracle's regenerated literal twiddles equal the decimal literals the
 reference spells out in src/kernels/dit.rs and src/kernels/codelets.rs.
 
-Runs only where /root/reference exists (the dev container).  It *reads* the reference
-source to compare numbers; nothing is copied into the repo.  Result is recorded in
-DESIGN.md; tests/test_oracle_literals.py runs it when the reference is present.
+The numbers are parsed from a checkout of the reference and stored, as data, in
+tests/golden/reference_literal_twiddles.npz (nothing else of the reference is kept);
+tests/test_oracle.py compares the oracle against that file, so the check needs no reference
+checkout.  Result is recorded in DESIGN.md.
 
-Usage: python oracle/check_literals.py [/root/reference]
+Usage: python oracle/check_literals.py REFERENCE_ROOT                  # compare against the sources
+       python oracle/check_literals.py REFERENCE_ROOT --write-golden   # (re)write the stored tables
 """
 from __future__ import annotations
 
@@ -18,6 +20,9 @@ import numpy as np
 
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from oracle import oracle as O  # noqa: E402
+
+GOLDEN = Path(__file__).resolve().parent.parent / "tests" / "golden" / "reference_literal_twiddles.npz"
+SOURCES = ("src/kernels/dit.rs", "src/kernels/codelets.rs")
 
 _FN = re.compile(r"fn\s+(fft_dit_chunk_(\d+)_simd_(f32|f64)|fft_dit_codelet_(\d+)_simd_(f32|f64))\s*<")
 _ARR = re.compile(r"let\s+(\w+)\s*=\s*(f32|f64)x(\d+)::simd_from\(\s*simd,\s*\[(.*?)\]\s*,?\s*\)", re.S)
@@ -62,17 +67,14 @@ def collect(path: Path):
             yield name, var, ty, vals
 
 
-def expected(chunk: int, ty: str):
-    return O.literal_twiddles(chunk, np.float32 if ty == "f32" else np.float64)
-
-
-def check(reference_root: str = "/root/reference") -> int:
+def tables(reference_root: str):
+    """Every literal table of the reference as (source, function, array, dtype, chunk, part, first index, values):
+    the table holds W_chunk^k for k = first index, first index + 1, ..., real part (part "re") or imaginary part ("im")."""
     root = Path(reference_root)
-    n_checked = 0
-    failures = []
-    for rel in ("src/kernels/dit.rs", "src/kernels/codelets.rs"):
+    out = []
+    for rel in SOURCES:
         for fn, var, ty, vals in collect(root / rel):
-            is_im = "_im" in var or var.endswith("im")
+            part = "im" if "_im" in var or var.endswith("im") else "re"
             m = re.search(r"_(\d+)_(\d+)$", var)
             lo = int(m.group(1)) if m else 0
             # which W_chunk table is it?  chunk kernels: from the function name; codelets: from the var/lanes
@@ -88,12 +90,38 @@ def check(reference_root: str = "/root/reference") -> int:
                     chunk = 16 if var in ("tw_re", "tw_im") else 32
                 if "_hi_" in var:
                     lo = chunk // 4
-            ere, eim = expected(chunk, ty)
-            exp = (eim if is_im else ere)[lo:lo + len(vals)]
-            got = np.array(vals, dtype=exp.dtype)
-            n_checked += len(vals)
-            if not np.array_equal(got, exp):
-                failures.append((rel, fn, var, got, exp))
+            out.append((rel, fn, var, ty, chunk, part, lo, np.array(vals, dtype=np.float32 if ty == "f32" else np.float64)))
+    return out
+
+
+def write_golden(reference_root: str, path: Path = GOLDEN) -> None:
+    tabs = tables(reference_root)
+    index = np.array([[rel, fn, var, ty, str(chunk), part, str(lo)] for rel, fn, var, ty, chunk, part, lo, _ in tabs])
+    np.savez_compressed(path, index=index, **{f"values_{i:03d}": t[-1] for i, t in enumerate(tabs)})
+    print(f"wrote {sum(t[-1].size for t in tabs)} literal twiddles of {len(tabs)} tables to {path}")
+
+
+def load_golden(path: Path = GOLDEN):
+    g = np.load(path)
+    return [(rel, fn, var, ty, int(chunk), part, int(lo), g[f"values_{i:03d}"])
+            for i, (rel, fn, var, ty, chunk, part, lo) in enumerate(g["index"])]
+
+
+def compare(tabs):
+    """(number of literals checked, tables that differ from the oracle's regenerated twiddles)."""
+    n_checked = 0
+    failures = []
+    for rel, fn, var, ty, chunk, part, lo, got in tabs:
+        ere, eim = O.literal_twiddles(chunk, np.float32 if ty == "f32" else np.float64)
+        exp = (eim if part == "im" else ere)[lo:lo + got.size]
+        n_checked += got.size
+        if got.dtype != exp.dtype or not np.array_equal(got, exp):
+            failures.append((rel, fn, var, got, exp))
+    return n_checked, failures
+
+
+def check(reference_root: str) -> int:
+    n_checked, failures = compare(tables(reference_root))
     for f in failures:
         print("MISMATCH", *f, sep="\n  ")
     print(f"checked {n_checked} literal twiddles against {reference_root}: "
@@ -102,4 +130,8 @@ def check(reference_root: str = "/root/reference") -> int:
 
 
 if __name__ == "__main__":
-    sys.exit(check(*(sys.argv[1:2])))
+    if len(sys.argv) < 2:
+        sys.exit(__doc__)
+    if "--write-golden" in sys.argv[2:]:
+        write_golden(sys.argv[1])
+    sys.exit(check(sys.argv[1]))

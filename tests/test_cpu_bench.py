@@ -31,6 +31,24 @@ def test_traffic_table_is_json_with_sources():
     json.dumps(table)
 
 
+def test_dump_sample_is_fixed_and_bounded(tmp_path):
+    """--dump-outputs: short arrays whole, long ones as the same seeded sample of elements in every run, at most 64 MiB in all."""
+    import numpy as np
+    import pytest
+    import torch
+    import bench
+    short = torch.arange(1000, dtype=torch.float64)
+    assert np.array_equal(bench.dump_sample(short), short.numpy())
+    long = torch.arange(1 << 23, dtype=torch.float64)
+    a, b = bench.dump_sample(long), bench.dump_sample(long.clone())
+    assert a.size == bench.DUMP_MAX_ELEMS and np.array_equal(a, b)
+    assert np.all(np.diff(a) > 0) and a[-1] < long.numel()           # distinct elements, in index order
+    bench.write_dump(tmp_path / "d", {"x": a, "y": a.astype(np.float32)})
+    assert np.array_equal(np.load(tmp_path / "d" / "x.npy"), a) and np.load(tmp_path / "d" / "y.npy").dtype == np.float32
+    with pytest.raises(AssertionError):
+        bench.write_dump(tmp_path / "e", {f"x{i}": a for i in range(5)})   # 5 x 16 MiB
+
+
 def test_criterion_writer_matches_the_overlay_scripts_reader(tmp_path):
     """tools/sweep.py --criterion writes what benches/plot_criterion_overlay.py reads: <group>/<series>/<n>/new/sample.json with
     per-sample iters and total times (ns) and benchmark.json with throughput ElementsAndBytes (benches/common/mod.rs:91-105)."""
