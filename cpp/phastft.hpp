@@ -65,6 +65,9 @@ template <> struct Api<double> {
     static void r2c_destroy(R2c* p) { phastft_plan_r2c_f64_destroy(p); }
     static int32_t r2c_host(const R2c* p, const double* in, std::size_t li, double* ore, std::size_t lre, double* oim, std::size_t lim) { return phastft_r2c_f64_host(p, in, li, ore, lre, oim, lim); }
     static int32_t c2r_host(const R2c* p, const double* ire, std::size_t lre, const double* iim, std::size_t lim, double* out, std::size_t lo, double* sre, std::size_t lsr, double* sim, std::size_t lsi) { return phastft_c2r_f64_host(p, ire, lre, iim, lim, out, lo, sre, lsr, sim, lsi); }
+    static int32_t r2c_reserve(const R2c* p, std::size_t b) { return phastft_plan_r2c_f64_reserve(p, b); }
+    static int32_t r2c_dev_batch(const R2c* p, const double* in, double* ore, double* oim, std::size_t b, std::size_t is, std::size_t os, void* s) { return phastft_r2c_f64_dev_batch(p, in, ore, oim, b, is, os, s); }
+    static int32_t c2r_dev_batch(const R2c* p, const double* ire, const double* iim, double* out, std::size_t b, std::size_t is, std::size_t os, void* s) { return phastft_c2r_f64_dev_batch(p, ire, iim, out, b, is, os, s); }
 };
 template <> struct Api<float> {
     using Dit = phastft_plan_dit_f32; using R2c = phastft_plan_r2c_f32;
@@ -82,6 +85,9 @@ template <> struct Api<float> {
     static void r2c_destroy(R2c* p) { phastft_plan_r2c_f32_destroy(p); }
     static int32_t r2c_host(const R2c* p, const float* in, std::size_t li, float* ore, std::size_t lre, float* oim, std::size_t lim) { return phastft_r2c_f32_host(p, in, li, ore, lre, oim, lim); }
     static int32_t c2r_host(const R2c* p, const float* ire, std::size_t lre, const float* iim, std::size_t lim, float* out, std::size_t lo, float* sre, std::size_t lsr, float* sim, std::size_t lsi) { return phastft_c2r_f32_host(p, ire, lre, iim, lim, out, lo, sre, lsr, sim, lsi); }
+    static int32_t r2c_reserve(const R2c* p, std::size_t b) { return phastft_plan_r2c_f32_reserve(p, b); }
+    static int32_t r2c_dev_batch(const R2c* p, const float* in, float* ore, float* oim, std::size_t b, std::size_t is, std::size_t os, void* s) { return phastft_r2c_f32_dev_batch(p, in, ore, oim, b, is, os, s); }
+    static int32_t c2r_dev_batch(const R2c* p, const float* ire, const float* iim, float* out, std::size_t b, std::size_t is, std::size_t os, void* s) { return phastft_c2r_f32_dev_batch(p, ire, iim, out, b, is, os, s); }
 };
 
 /// planner.rs:34-114
@@ -116,6 +122,8 @@ class PlannerR2c {
     PlannerR2c(const PlannerR2c&) = delete;
     PlannerR2c& operator=(const PlannerR2c&) = delete;
     const typename Api<T>::R2c* raw() const { return raw_; }
+    /// additive: size the half-length transform's workspace for batched calls of up to `batch` members now
+    void reserve(std::size_t batch) const { check(Api<T>::r2c_reserve(raw_, batch)); }
   private:
     typename Api<T>::R2c* raw_ = nullptr;
 };
@@ -165,6 +173,20 @@ inline void fft_64_dit_device(double* d_reals, double* d_imags, Direction d, con
 }
 inline void fft_32_dit_device(float* d_reals, float* d_imags, Direction d, const PlannerDit32& p, std::size_t batch, std::size_t batch_stride, void* stream) {
     check(detail::Api<float>::fft_dev(p.raw(), d_reals, d_imags, (int)d, batch, batch_stride, stream));
+}
+/// Batched device-resident r2c / c2r (phastft_{r2c,c2r}_*_dev_batch): strides in elements; the real-side stride even and
+/// its base aligned to two elements.
+inline void r2c_fft_f64_device_batch(const double* d_in, double* d_out_re, double* d_out_im, const PlannerR2c64& p, std::size_t batch, std::size_t in_stride, std::size_t out_stride, void* stream) {
+    check(detail::Api<double>::r2c_dev_batch(p.raw(), d_in, d_out_re, d_out_im, batch, in_stride, out_stride, stream));
+}
+inline void r2c_fft_f32_device_batch(const float* d_in, float* d_out_re, float* d_out_im, const PlannerR2c32& p, std::size_t batch, std::size_t in_stride, std::size_t out_stride, void* stream) {
+    check(detail::Api<float>::r2c_dev_batch(p.raw(), d_in, d_out_re, d_out_im, batch, in_stride, out_stride, stream));
+}
+inline void c2r_fft_f64_device_batch(const double* d_in_re, const double* d_in_im, double* d_out, const PlannerR2c64& p, std::size_t batch, std::size_t in_stride, std::size_t out_stride, void* stream) {
+    check(detail::Api<double>::c2r_dev_batch(p.raw(), d_in_re, d_in_im, d_out, batch, in_stride, out_stride, stream));
+}
+inline void c2r_fft_f32_device_batch(const float* d_in_re, const float* d_in_im, float* d_out, const PlannerR2c32& p, std::size_t batch, std::size_t in_stride, std::size_t out_stride, void* stream) {
+    check(detail::Api<float>::c2r_dev_batch(p.raw(), d_in_re, d_in_im, d_out, batch, in_stride, out_stride, stream));
 }
 
 // ---- r2c / c2r (algorithms/r2c.rs:521-895) --------------------------------------------------------------

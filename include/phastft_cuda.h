@@ -203,6 +203,31 @@ PHASTFT_API int32_t phastft_c2r_f64_dev(const phastft_plan_r2c_f64* plan, const 
 PHASTFT_API int32_t phastft_c2r_f32_dev(const phastft_plan_r2c_f32* plan, const float* d_in_re, const float* d_in_im,
                                         float* d_output, float* d_scratch_re, float* d_scratch_im, void* stream);
 
+/* ---- batched device-resident r2c / c2r (the reference has no batch API: a caller loop sharing one planner) --------
+ * Strides are in elements of T.
+ *   r2c: member b reads d_input[b*in_stride ..][..N] and writes bins [b*out_stride ..][..N/2+1] of both output planes
+ *        (in_stride >= N, out_stride >= N/2+1).
+ *   c2r: member b reads bins [b*in_stride ..][..N/2+1] of both input planes and writes d_output[b*out_stride ..][..N]
+ *        (in_stride >= N/2+1, out_stride >= N), normalised as phastft_c2r_*_dev.
+ * The real side is read or written as complex pairs: its stride must be even and its base pointer aligned to
+ * 2*sizeof(T), else PHASTFT_ERR_INVALID_ARG before anything is launched.  Padding between members and the spectrum input
+ * of c2r are never written.  Stream-ordered and asynchronous like the single-call entries, which batch == 1 runs.  No
+ * scratch: every batched c2r pre-processes the spectrum while its first kernel loads it.  Any batch count. */
+PHASTFT_API int32_t phastft_r2c_f64_dev_batch(const phastft_plan_r2c_f64* plan, const double* d_input, double* d_out_re,
+                                              double* d_out_im, size_t batch, size_t in_stride, size_t out_stride, void* stream);
+PHASTFT_API int32_t phastft_r2c_f32_dev_batch(const phastft_plan_r2c_f32* plan, const float* d_input, float* d_out_re,
+                                              float* d_out_im, size_t batch, size_t in_stride, size_t out_stride, void* stream);
+PHASTFT_API int32_t phastft_c2r_f64_dev_batch(const phastft_plan_r2c_f64* plan, const double* d_in_re, const double* d_in_im,
+                                              double* d_output, size_t batch, size_t in_stride, size_t out_stride, void* stream);
+PHASTFT_API int32_t phastft_c2r_f32_dev_batch(const phastft_plan_r2c_f32* plan, const float* d_in_re, const float* d_in_im,
+                                              float* d_output, size_t batch, size_t in_stride, size_t out_stride, void* stream);
+/* Sizes the workspace of the plan's half-length transform for batches of up to `batch` members now, as
+ * phastft_plan_dit_*_reserve does: a batched r2c / c2r can then be captured into a CUDA graph.  (With the opt-in
+ * pipelined two-pass launch, PHASTFT_PIPE=1, that launch's per-call counters are still allocated by the first
+ * uncaptured call, for c2c and r2c alike.) */
+PHASTFT_API int32_t phastft_plan_r2c_f64_reserve(const phastft_plan_r2c_f64* plan, size_t batch);
+PHASTFT_API int32_t phastft_plan_r2c_f32_reserve(const phastft_plan_r2c_f32* plan, size_t batch);
+
 /* ---- lib.rs:41-140 (feature complex-nums): fft_{64,32}_interleaved* --------------------------
  * signal = N interleaved (re, im) pairs (num_complex::Complex<T> layout), in place.  The
  * reference deinterleaves into two fresh Vecs, runs the planar FFT and re-interleaves

@@ -100,6 +100,9 @@ SIGNATURES = {
     "phastft_c2r_{s}_host": ([_vp, _vp, _sz, _vp, _sz, _vp, _sz, _vp, _sz, _vp, _sz], _i32),
     "phastft_c2r_{s}_oneshot": ([_vp, _sz, _vp, _sz, _vp, _sz, _ci], _i32),
     "phastft_c2r_{s}_dev": ([_vp, _vp, _vp, _vp, _vp, _vp, _vp], _i32),
+    "phastft_r2c_{s}_dev_batch": ([_vp, _vp, _vp, _vp, _sz, _sz, _sz, _vp], _i32),
+    "phastft_c2r_{s}_dev_batch": ([_vp, _vp, _vp, _vp, _sz, _sz, _sz, _vp], _i32),
+    "phastft_plan_r2c_{s}_reserve": ([_vp, _sz], _i32),
 }
 def check(code: int):
     if code != OK:

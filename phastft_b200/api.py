@@ -37,7 +37,7 @@ __all__ = [
     "c2r_fft_f64_with_planner_and_scratch",
     "r2c_fft_f32", "r2c_fft_f32_with_planner", "c2r_fft_f32", "c2r_fft_f32_with_planner",
     "c2r_fft_f32_with_planner_and_scratch",
-    "fft_dit_batch", "fft_dit_batch_sharded", "host_register", "host_unregister",
+    "fft_dit_batch", "fft_dit_batch_sharded", "r2c_fft_batch", "c2r_fft_batch", "host_register", "host_unregister",
 ]
 
 
@@ -186,6 +186,12 @@ class _PlannerR2c:
     @classmethod
     def new(cls, n: int, device: int = 0):
         return cls(n, device)
+
+    def reserve(self, batch: int) -> None:
+        """Size the workspace of the half-length transform for r2c_fft_batch / c2r_fft_batch calls of up to `batch`
+        members now (otherwise the first larger call grows it, synchronising the device -- an error inside a CUDA-graph
+        capture)."""
+        check(fn("phastft_plan_r2c_{s}_reserve", self._sfx)(self._h, int(batch)))
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -338,6 +344,37 @@ def fft_dit_batch_sharded(reals: np.ndarray, imags: np.ndarray, direction: Direc
         raise PhastFTPanic(13, "arrays shorter than batch * batch_stride")
     arr = (C.c_void_p * len(planners))(*[p._h for p in planners])
     check(fn("phastft_fft_dit_{s}_batch_sharded_host", sfx)(arr, len(planners), pr, pi, int(batch), stride, int(direction)))
+
+
+def _real_batch_args(x_real, planes, planner, batch, real_stride, spec_stride):
+    n, half = planner.n, planner.n // 2
+    real_stride = n if real_stride is None else int(real_stride)
+    spec_stride = half + 1 if spec_stride is None else int(spec_stride)
+    px, nx = _torch_ptr(x_real, planner._dtype)
+    (pa, na), (pb, nb) = (_torch_ptr(t, planner._dtype) for t in planes)
+    if batch < 1 or real_stride < n or spec_stride < half + 1:
+        raise PhastFTPanic(13, "batch >= 1, real-side stride >= N and spectrum stride >= N/2 + 1 required")
+    if nx < (batch - 1) * real_stride + n:
+        raise PhastFTPanic(13, "real tensor shorter than (batch - 1) * stride + N")
+    if min(na, nb) < (batch - 1) * spec_stride + half + 1:
+        raise PhastFTPanic(13, "spectrum tensors shorter than (batch - 1) * stride + N/2 + 1")
+    return px, pa, pb, real_stride, spec_stride
+
+
+def r2c_fft_batch(x, out_re, out_im, planner, batch: int, in_stride: int | None = None, out_stride: int | None = None) -> None:
+    """Batched device-resident r2c: member b reads x[b*in_stride:][:N] and writes bins out_re/out_im[b*out_stride:][:N/2+1]
+    (1-D contiguous torch CUDA tensors, strides in elements, defaults N and N/2+1).  in_stride must be even and x's start
+    aligned to two elements (the reals are read as complex pairs).  Asynchronous on torch's current stream."""
+    px, pr, pi, in_stride, out_stride = _real_batch_args(x, (out_re, out_im), planner, batch, in_stride, out_stride)
+    check(fn("phastft_r2c_{s}_dev_batch", planner._sfx)(planner._h, px, pr, pi, int(batch), in_stride, out_stride, _torch_stream(x)))
+
+
+def c2r_fft_batch(in_re, in_im, out, planner, batch: int, in_stride: int | None = None, out_stride: int | None = None) -> None:
+    """Batched device-resident c2r, the inverse of r2c_fft_batch: member b reads bins in_re/in_im[b*in_stride:][:N/2+1]
+    (not modified) and writes out[b*out_stride:][:N], normalised so that c2r(r2c(x)) == x.  out_stride must be even and
+    out's start aligned to two elements.  No scratch."""
+    po, pr, pi, out_stride, in_stride = _real_batch_args(out, (in_re, in_im), planner, batch, out_stride, in_stride)
+    check(fn("phastft_c2r_{s}_dev_batch", planner._sfx)(planner._h, pr, pi, po, int(batch), in_stride, out_stride, _torch_stream(out)))
 
 
 def host_register(array: np.ndarray) -> None:

@@ -71,8 +71,10 @@ struct PassParams {
     int in_ring;                   // KIND_TRANS: applied to the batch index of the INPUT address
     // c2r pre-processing on load (MODE_C2R_IN only): in_re / in_im are the N/2 + 1 bins of the half-spectrum, the pass's
     // input element k is built from bins k and N/2 - k with the twiddle W_N^k out of this table
+    // (MODE_R2C_OUT: the same W_N table, for the untangle of the one-CTA kernel's result)
     Tw2 pre_tw2;
     int pre_log2half;              // log2(N/2); 0 = no pre-processing
+    int r2c_out;                   // host only: launch the MODE_R2C_OUT build of the one-CTA kernel
     double2 pre_wc[32];            // W_(2 R1)^i, i < R1 = the kernel's first radix
     // TMA tile input (MODE_TMA_IN only): one tensor map per planar array, dims {B columns, R rows, batch}
     alignas(64) CUtensorMap tmap_re;
@@ -106,6 +108,48 @@ struct TileAddr {
         }
     }
 };
+
+// ---------------------------------------------------------------------------------------------
+// r2c / c2r arithmetic, the one copy: called by the elementwise kernels at the end of this file and by the pass kernels that
+// fold it into their loads (MODE_C2R_IN) or their last store (MODE_R2C_OUT).  c_h + i s_h = wkr + i wki = 0.5 * W_N^k.
+// ---------------------------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ void half_twiddle(const Tw2& tw2, uint32_t k, T& c_h, T& s_h) {
+    const double2 wd = tw2.get(k);
+    c_h = T(0.5 * wd.x); s_h = T(0.5 * wd.y);
+}
+// r2c untangle of bin 0 (r2c.rs:161-166): Z[0] = (a0 + i b0) in, the real bins X[0] and X[N/2] out
+template <typename T>
+__device__ __forceinline__ void r2c_untangle_ends(T a0, T b0, T& r0, T& rh) {
+    r0 = a0 + b0; rh = a0 - b0;
+}
+// r2c untangle of the self pair k = N/4 (r2c.rs:233-236): Z[N/4] = (a + ib) in, X[N/4] out
+template <typename T>
+__device__ __forceinline__ void r2c_untangle_self(T a, T b, T wkr, T wki, T& rq, T& iq) {
+    rq = a + T(2) * wkr * b;
+    iq = T(2) * wki * b;
+}
+// r2c untangle of the bin pair (k, m = N/2 - k), k != 0, N/4 (r2c.rs:167-232): (a + ib) = Z[k], (c + id) = Z[m] of the
+// half-length transform in, X[k] and X[m] out
+template <typename T>
+__device__ __forceinline__ void r2c_untangle_pair(T a, T b, T c, T d, T wkr, T wki, T& rk, T& ik, T& rm, T& im) {
+    T s_re = T(0.5) * (a + c), s_im = T(0.5) * (b - d);
+    T t_re = b + d, t_im = c - a;
+    T wzr = wkr * t_re - wki * t_im;
+    T wzi = wkr * t_im + wki * t_re;
+    rk = s_re + wzr; ik = s_im + wzi;
+    rm = s_re - wzr; im = wzi - s_im;
+}
+// c2r pre-processing of element k (r2c.rs:263-347): bins k = (re_f + i im_f) and conj(bin N/2 - k) = (re_s + i im_s) in,
+// element k of the half-length inverse transform's input out
+template <typename T>
+__device__ __forceinline__ cx<T> c2r_element(T re_f, T im_f, T re_s, T im_s, T c_h, T s_h) {
+    T zx_re = T(0.5) * (re_f + re_s), zx_im = T(0.5) * (im_f + im_s);
+    T dr = re_f - re_s, di = im_f - im_s;
+    T zy_re = c_h * dr + s_h * di;
+    T zy_im = c_h * di - s_h * dr;
+    return make_cx<T>(zx_re - zy_im, zx_im + zy_re);
+}
 
 // ---------------------------------------------------------------------------------------------
 // The pass kernel.
@@ -182,7 +226,12 @@ __device__ __forceinline__ void bulk_load_1d(unsigned smem_dst, const void* gsrc
 //      last stage writes its results into a second planar staging area and two cp.async.bulk copies take them out.  The
 //      per-lane 4/8-byte accesses of the plain kernel (128 bytes per f32 warp instruction, the bound of the 16..128-point
 //      batches) become two asynchronous copies per CTA.
-enum { MODE_PLAIN = 0, MODE_XCH_PRODUCE = 1, MODE_XCH_CONSUME = 2, MODE_TMA_IN = 3, MODE_BULK_IN = 4, MODE_C2R_IN = 5, MODE_ROW_BULK = 6 };
+//   7  r2c untangle on store (KIND_ROW, batched r2c): the row is a member's N reals read as N/2 complex pairs; the last stage
+//      puts its results back into the tile, and after a barrier each thread takes one bin pair (k, N/2 - k) of one member out
+//      of shared memory and stores the untangled bins N/2 + 1 straight to the planar outputs.  The separate untangle sweep
+//      and its HBM round trip disappear.
+enum { MODE_PLAIN = 0, MODE_XCH_PRODUCE = 1, MODE_XCH_CONSUME = 2, MODE_TMA_IN = 3, MODE_BULK_IN = 4, MODE_C2R_IN = 5, MODE_ROW_BULK = 6,
+       MODE_R2C_OUT = 7 };
 template <typename T, class RL, int C, int NT, int KIND, int XCH = 0, int VARIANT = 0>
 struct PassKernel {
     static constexpr int S = RL::S;
@@ -201,7 +250,8 @@ struct PassKernel {
     static constexpr size_t MBAR_OFF = (TABLE_END + 15) & ~size_t(15);
     static constexpr size_t OUT_OFF = (MBAR_OFF + 16 + 127) & ~size_t(127);      // MODE_ROW_BULK: planar output staging [2][C][R]
     static constexpr size_t SMEM_BYTES = XCH == MODE_ROW_BULK ? OUT_OFF + sizeof(cx<T>) * (size_t)TILE_ELEMS : ASYNC_IN ? MBAR_OFF + 16 : TABLE_END;
-    static_assert(XCH == 0 || S >= 2, "an exchanging pass needs a shared-memory tile");
+    static_assert(XCH == 0 || XCH == MODE_C2R_IN || S >= 2, "an exchanging pass needs a shared-memory tile");
+    static_assert(XCH != MODE_R2C_OUT || KIND == KIND_ROW, "r2c untangle on store: one-CTA kernels");
     static_assert(XCH != 1 || KIND == KIND_COL, "the producer of a cluster exchange is a COL pass");
     static_assert(XCH != 2 || KIND == KIND_TRANS, "the consumer of a cluster exchange is a TRANS pass");
     static_assert(XCH != MODE_TMA_IN || (KIND == KIND_COL && C * sizeof(T) >= 16), "TMA tile input: COL pass, rows of >= 16 bytes");
@@ -239,16 +289,17 @@ struct PassKernel {
     // (same arithmetic, in the same order, as c2r_preprocess_kernel below; r2c.rs:263-347).  The inverse runs as a forward
     // transform of the swapped parts (r2c.rs:782), so the kernel is handed (im, re).
     template <int N>
-    static __device__ __forceinline__ void gload_c2r(const PassParams<T>& p, long long a0, long long step, cx<T> (&x)[N]) {
-        // element i is bin k = a0 + i * step with step = (N/2) / R1 (first pass: R * B = N/2), so its twiddle
-        // W_N^k = W_N^a0 * W_(2 R1)^i: one table lookup per task, the second factors are launch constants (pre_wc).
+    static __device__ __forceinline__ void gload_c2r(const PassParams<T>& p, long long mb, long long k0, long long step, cx<T> (&x)[N]) {
+        // mb: the member's first bin in in_re / in_im; element i is bin k = k0 + i * step of that member, with
+        // step = (N/2) / R1 (first pass: R * B = N/2; one-CTA kernel: M = R / R1), so its twiddle
+        // W_N^k = W_N^k0 * W_(2 R1)^i: one table lookup per task, the second factors are launch constants (pre_wc).
         // Loads in groups of 8 (f64): 4 scalars per element, all of a group in flight at once.
         const long long half = 1LL << p.pre_log2half;
-        const T* __restrict__ fr = p.in_re + a0;
-        const T* __restrict__ fi = p.in_im + a0;
-        const T* __restrict__ sr = p.in_re + (half - a0);
-        const T* __restrict__ si = p.in_im + (half - a0);
-        const double2 wb = p.pre_tw2.get((uint32_t)a0);
+        const T* __restrict__ fr = p.in_re + mb + k0;
+        const T* __restrict__ fi = p.in_im + mb + k0;
+        const T* __restrict__ sr = p.in_re + mb + (half - k0);
+        const T* __restrict__ si = p.in_im + mb + (half - k0);
+        const double2 wb = p.pre_tw2.get((uint32_t)k0);
         constexpr int G = (sizeof(T) == 8 && N > 8) ? 8 : N;
 #pragma unroll
         for (int g0 = 0; g0 < N; g0 += G) {
@@ -263,18 +314,17 @@ struct PassKernel {
             for (int i = 0; i < G; ++i) {
                 const double2 wd = (g0 + i == 0) ? wb : cmul_d(wb, p.pre_wc[g0 + i]);
                 const T c_h = T(0.5 * wd.x), s_h = T(0.5 * wd.y);
-                const T zx_re = T(0.5) * (re_f[i] + re_s[i]), zx_im = T(0.5) * (im_f[i] + im_s[i]);
-                const T dr = re_f[i] - re_s[i], di = im_f[i] - im_s[i];
-                const T zy_re = c_h * dr + s_h * di;
-                const T zy_im = c_h * di - s_h * dr;
-                x[g0 + i] = make_cx<T>(zx_im + zy_re, zx_re - zy_im);
+                const cx<T> z = c2r_element<T>(re_f[i], im_f[i], re_s[i], im_s[i], c_h, s_h);
+                x[g0 + i] = make_cx<T>(z.y, z.x);
             }
         }
     }
+    // mb (MODE_C2R_IN only): offset of the element's batch member, a0 - mb its index inside the member
     template <int N, int IL = -1>
-    static __device__ __forceinline__ void gload_n(const PassParams<T>& p, long long a0, long long step, cx<T> (&x)[N]) {
+    static __device__ __forceinline__ void gload_n(const PassParams<T>& p, long long a0, long long step, cx<T> (&x)[N],
+                                                   [[maybe_unused]] long long mb = 0) {
         if constexpr (XCH == MODE_C2R_IN) {
-            gload_c2r<N>(p, a0, step, x);
+            gload_c2r<N>(p, mb, a0 - mb, step, x);
         } else if constexpr (IL < 0) {
             if (p.in_interleaved == 0) gload_n<N, 0>(p, a0, step, x);
             else if (p.in_interleaved == 1) gload_n<N, 1>(p, a0, step, x);
@@ -386,7 +436,8 @@ struct PassKernel {
 #endif
             }
             DftC<T, RAD>::run(x);
-            if constexpr (!LAST) {
+            if constexpr (!LAST || XCH == MODE_R2C_OUT) {
+                // (MODE_R2C_OUT: the last stage's outputs kr = m + k*NS go back to their natural positions for the untangle)
 #pragma unroll
                 for (int k = 0; k < RAD; ++k) tile[Addr::at(base + k * NS, c)] = x[k];
             } else if constexpr (XCH == 1) {
@@ -466,6 +517,7 @@ struct PassKernel {
         uint32_t kp0 = 0;              // previous-pass output digit of column c = 0
         uint32_t kp_cstep = 0;         // ... and its increment per column
         uint32_t bcol0 = 0;            // flat index of the remaining digits for column 0 (COL only)
+        [[maybe_unused]] long long in_mbase = 0;   // COL, MODE_C2R_IN: first element of the tile's batch member
 
         if constexpr (KIND == KIND_COL) {
             const int tilesB = 1 << (p.log2B - LOG2C);
@@ -475,7 +527,8 @@ struct PassKernel {
             const int a = rest & ((1 << p.log2A) - 1);
             const int batch = rest >> p.log2A;
             const long long off = ((long long)a << (LOG2R + p.log2B)) + ((long long)bt << LOG2C);
-            in_base = (long long)batch * p.in_bstride + off;
+            in_mbase = (long long)batch * p.in_bstride;
+            in_base = in_mbase + off;
             out_base = (long long)(p.out_ring ? (batch & (p.out_ring - 1)) : batch) * p.out_bstride + off;
             in_rstride = 1LL << p.log2B;
             in_cstride = 1;
@@ -570,7 +623,8 @@ struct PassKernel {
                     for (int i = 0; i < R1; ++i) pre[i] = src[i * M];
                 } else if ((KIND != KIND_ROW) || (c < rows_valid)) {
                     const long long a0 = in_base + (long long)c * in_cstride + (long long)mp * in_rstride;
-                    gload_n<R1>(p, a0, (long long)M * in_rstride, pre);
+                    const long long mb = (KIND == KIND_ROW) ? in_base + (long long)c * in_cstride : in_mbase;
+                    gload_n<R1>(p, a0, (long long)M * in_rstride, pre, mb);
                 } else {
 #pragma unroll
                     for (int i = 0; i < R1; ++i) pre[i] = make_cx<T>(T(0), T(0));
@@ -659,7 +713,8 @@ struct PassKernel {
                     for (int i = 0; i < R1; ++i) x[i] = pre[i];
                 } else if (valid) {
                     const long long a0 = in_base + (long long)c * in_cstride + (long long)mp * in_rstride;
-                    gload_n<R1, IL>(p, a0, (long long)M * in_rstride, x);
+                    const long long mb = (KIND == KIND_ROW) ? in_base + (long long)c * in_cstride : in_mbase;
+                    gload_n<R1, IL>(p, a0, (long long)M * in_rstride, x, mb);
                 } else {
 #pragma unroll
                     for (int i = 0; i < R1; ++i) x[i] = make_cx<T>(T(0), T(0));
@@ -695,6 +750,35 @@ struct PassKernel {
         else stage1(std::integral_constant<int, 2>{});
         // ---- stages 2..S -------------------------------------------------------------------------
         run_stages<1>(p, tile, out_base, out_kstride, rows_valid, tid);
+        if constexpr (XCH == MODE_R2C_OUT) {
+            // Z = the tile's row c (the half-length transform of member c's reals as pairs).  Task (c, k), k < R/2: bins k and
+            // R - k; k == 0 also does bins 0, R and the self pair R/2 (as r2c_untangle_kernel).  Consecutive lanes take
+            // consecutive k, so the stores of bins k (ascending) and R - k (descending) are both warp-contiguous.
+            __syncthreads();
+            constexpr int Q = R / 2;
+            for (int t = tid; t < C * Q; t += NT) {
+                const int c = t / Q, k = t % Q;
+                if (c >= rows_valid) break;
+                T* ore = p.out_re + out_base + (long long)c * p.out_bstride;
+                T* oim = p.out_im + out_base + (long long)c * p.out_bstride;
+                if (k == 0) {
+                    const cx<T> z0 = tile[Addr::at(0, c)];
+                    T r0, rh;
+                    r2c_untangle_ends<T>(z0.x, z0.y, r0, rh);
+                    ore[0] = r0; oim[0] = T(0);
+                    ore[R] = rh; oim[R] = T(0);
+                    T wkr, wki;
+                    half_twiddle<T>(p.pre_tw2, (uint32_t)Q, wkr, wki);
+                    const cx<T> zq = tile[Addr::at(Q, c)];
+                    r2c_untangle_self<T>(zq.x, zq.y, wkr, wki, ore[Q], oim[Q]);
+                } else {
+                    T wkr, wki;
+                    half_twiddle<T>(p.pre_tw2, (uint32_t)k, wkr, wki);
+                    const cx<T> zk = tile[Addr::at(k, c)], zm = tile[Addr::at(R - k, c)];
+                    r2c_untangle_pair<T>(zk.x, zk.y, zm.x, zm.y, wkr, wki, ore[k], oim[k], ore[R - k], oim[R - k]);
+                }
+            }
+        }
         if constexpr (XCH == MODE_ROW_BULK) {
             // the staging area was written through the generic proxy: make it visible to the asynchronous proxy, then one thread
             // copies the two planes out and waits until the copies have READ shared memory before the CTA may exit
@@ -717,7 +801,7 @@ template <typename T, class RL, int C, int NT, int KIND, int VARIANT = 0, int MI
 __global__ void __launch_bounds__(NT, MINB) fft_pass_kernel(const __grid_constant__ PassParams<T> p) {
     PassKernel<T, RL, C, NT, KIND, 0, VARIANT>::body(p, blockIdx.x);
 }
-// the same pass with an asynchronous tile input (MODE_TMA_IN / MODE_BULK_IN)
+// the same pass with an asynchronous tile input (MODE_TMA_IN / MODE_BULK_IN) or another MODE_* of its loads / stores
 template <typename T, class RL, int C, int NT, int KIND, int MODE, int VARIANT = 0, int MINB = 0>
 __global__ void __launch_bounds__(NT, MINB) fft_pass_async_kernel(const __grid_constant__ PassParams<T> p) {
     PassKernel<T, RL, C, NT, KIND, MODE, VARIANT>::body(p, blockIdx.x);
@@ -840,6 +924,29 @@ struct RealParams {
     Tw2 tw2;                    // two-level table for W_N, N = 2*half
 };
 
+// Bin pair k of one member (k <= N/4; k == 0 also does bin N/2), in place on its half+1 slots.
+template <typename T>
+__device__ __forceinline__ void r2c_untangle_at(T* re, T* im, long long k, long long half, const Tw2& tw2) {
+    const long long q = half >> 1;
+    if (k == 0) {
+        T a0 = re[0], b0 = im[0], r0, rh;
+        r2c_untangle_ends<T>(a0, b0, r0, rh);
+        re[0] = r0; im[0] = T(0);
+        re[half] = rh; im[half] = T(0);
+        return;
+    }
+    T wkr, wki;
+    half_twiddle<T>(tw2, (uint32_t)k, wkr, wki);
+    if (k == q) {
+        T a = re[q], b = im[q];
+        r2c_untangle_self<T>(a, b, wkr, wki, re[q], im[q]);
+        return;
+    }
+    const long long m = half - k;
+    T a = re[k], b = im[k], c = re[m], d = im[m];
+    r2c_untangle_pair<T>(a, b, c, d, wkr, wki, re[k], im[k], re[m], im[m]);
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256) r2c_untangle_kernel(const __grid_constant__ RealParams<T> p) {
     const long long half = 1LL << p.log2half;
@@ -848,30 +955,19 @@ __global__ void __launch_bounds__(256) r2c_untangle_kernel(const __grid_constant
     T* re = p.re + (long long)blockIdx.y * p.bstride;
     T* im = p.im + (long long)blockIdx.y * p.bstride;
     if (k > q) return;
-    if (k == 0) {
-        // r2c.rs:161-166
-        T a0 = re[0], b0 = im[0];
-        re[0] = a0 + b0; im[0] = T(0);
-        re[half] = a0 - b0; im[half] = T(0);
-        return;
-    }
-    double2 wd = p.tw2.get((uint32_t)k);
-    const T wkr = T(0.5 * wd.x), wki = T(0.5 * wd.y);
-    if (k == q) {
-        // r2c.rs:233-236 (self pair)
-        T a = re[q], b = im[q];
-        re[q] = a + T(2) * wkr * b;
-        im[q] = T(2) * wki * b;
-        return;
-    }
-    const long long m = half - k;
-    T a = re[k], b = im[k], c = re[m], d = im[m];
-    T s_re = T(0.5) * (a + c), s_im = T(0.5) * (b - d);
-    T t_re = b + d, t_im = c - a;
-    T wzr = wkr * t_re - wki * t_im;
-    T wzi = wkr * t_im + wki * t_re;
-    re[k] = s_re + wzr; im[k] = s_im + wzi;
-    re[m] = s_re - wzr; im[m] = wzi - s_im;
+    r2c_untangle_at<T>(re, im, k, half, p.tw2);
+}
+
+// The same untangle over `members` members of a batch with the (member, k) pairs flattened into grid.x: every thread has
+// work whatever N is (r2c_untangle_kernel gives each member whole 256-thread blocks, of which N/4 + 1 threads are active).
+template <typename T>
+__global__ void __launch_bounds__(256) r2c_untangle_batch_kernel(const __grid_constant__ RealParams<T> p, long long members) {
+    const long long half = 1LL << p.log2half;
+    const long long q1 = (half >> 1) + 1;            // pairs k = 0 .. N/4 per member
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= members * q1) return;
+    const long long b = g / q1, k = g - b * q1;
+    r2c_untangle_at<T>(p.re + b * p.bstride, p.im + b * p.bstride, k, half, p.tw2);
 }
 
 template <typename T>
@@ -884,17 +980,14 @@ __global__ void __launch_bounds__(256) c2r_preprocess_kernel(const __grid_consta
     T* zre = p.re + (long long)blockIdx.y * p.bstride;
     T* zim = p.im + (long long)blockIdx.y * p.bstride;
     const long long m = half - k;
-    double2 wd = p.tw2.get((uint32_t)k);
-    const T c_h = T(0.5 * wd.x), s_h = T(0.5 * wd.y);
+    T c_h, s_h;
+    half_twiddle<T>(p.tw2, (uint32_t)k, c_h, s_h);
     // r2c.rs:263-347
     T re_f = ire[k], im_f = iim[k];
     T re_s = ire[m], im_s = -iim[m];
-    T zx_re = T(0.5) * (re_f + re_s), zx_im = T(0.5) * (im_f + im_s);
-    T dr = re_f - re_s, di = im_f - im_s;
-    T zy_re = c_h * dr + s_h * di;
-    T zy_im = c_h * di - s_h * dr;
-    zre[k] = zx_re - zy_im;
-    zim[k] = zx_im + zy_re;
+    const cx<T> z = c2r_element<T>(re_f, im_f, re_s, im_s, c_h, s_h);
+    zre[k] = z.x;
+    zim[k] = z.y;
 }
 
 }  // namespace phast

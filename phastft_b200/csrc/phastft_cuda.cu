@@ -186,6 +186,9 @@ struct PassDesc {
     const KernelEntry<T>* kb = nullptr;   // kernel when the call carries many transforms (multi-wave grids)
     const KernelEntry<T>* kt = nullptr;   // 2-pass plans of lone transforms: the pass with an asynchronous (TMA) tile input
     const KernelEntry<T>* kc = nullptr;   // first pass only: `k` with the c2r pre-processing folded into its loads (MODE_C2R_IN)
+    const KernelEntry<T>* kcb = nullptr;  // ... the same for batched c2r calls: `kb`'s build (first COL pass: any build of the same R)
+    const KernelEntry<T>* kf = nullptr;   // one-CTA kernels: `k` / `kb` with the r2c untangle on store (MODE_R2C_OUT), if they have
+    const KernelEntry<T>* kfb = nullptr;  // a shared-memory stage
     const KernelEntry<T>* kr = nullptr;   // one-CTA plans: `kb` with its tile moved in and out by cp.async.bulk (MODE_ROW_BULK)
     size_t tw_wc_off_t = (size_t)-1;      // W_L^(c*m) table for `kt`
     size_t tw_im_off = (size_t)-1;        // one-CTA kernels: the per-stage [i][m] stage-twiddle tables for `k` ...
@@ -436,6 +439,22 @@ const KernelEntry<T>* find_row_bulk(const KernelEntry<T>* kb) {
     return nullptr;
 }
 
+// The build of `k`'s tile (same kind, radices, C, NT and id) with the given MODE_*, or NULL (the last registered, if several).
+template <typename T>
+const KernelEntry<T>* find_mode(const KernelEntry<T>* k, int mode) {
+    const KernelEntry<T>* found = nullptr;
+    if (!k) return found;
+    for (const auto& e : registry<T>())
+        if (e.mode == mode && e.kind == k->kind && e.R == k->R && e.C == k->C && e.NT == k->NT && e.variant == k->variant && e.rl == k->rl) found = &e;
+    return found;
+}
+// the MODE_C2R_IN / MODE_R2C_OUT builds of a one-CTA pass's kernels (batched real transforms)
+template <typename T>
+void find_real_modes(PassDesc<T>& d) {
+    d.kc = find_mode(d.k, MODE_C2R_IN); d.kcb = find_mode(d.kb, MODE_C2R_IN);
+    d.kf = find_mode(d.k, MODE_R2C_OUT); d.kfb = find_mode(d.kb, MODE_R2C_OUT);
+}
+
 // Entries of the concatenated per-stage [i][m] stage-twiddle tables of a one-CTA kernel (stage q >= 1 owns Ns(q) * rad(q)).
 template <typename T>
 size_t tw_im_entries(const KernelEntry<T>* k) {
@@ -510,10 +529,14 @@ int32_t build_plan(size_t n, int device, Plan<T>** out) {
         d.kb = (kind == KIND_ROW) ? pick_row_batch_kernel<T>(1 << f[p], d.k) : pick_kernel<T>(kind, 1 << f[p], max_c, p, /*hbm_strided=*/wide_b, false, 0, pref_c_b, pref_v);
         if (!d.k) return fail(PHASTFT_ERR_INVALID_ARG, "no kernel for pass size 2^" + std::to_string(f[p]) + " kind " + kind_name(kind));
         if (kind == KIND_ROW) d.kr = find_row_bulk<T>(d.kb);
-        if (p == 0 && kind == KIND_COL)         // the same tile with the c2r pre-processing in its loads, if compiled (c2r_dev uses it)
+        if (kind == KIND_ROW) find_real_modes(d);
+        if (p == 0 && kind == KIND_COL) {       // the same tile with the c2r pre-processing in its loads, if compiled (c2r_dev uses it)
+            d.kc = find_mode(d.k, MODE_C2R_IN);
+            // batched c2r: no table of a first COL pass depends on its tile, so any build of the same R serves if kb has none
+            d.kcb = find_mode(d.kb, MODE_C2R_IN);
             for (const auto& e : registry<T>())
-                if (e.mode == MODE_C2R_IN && e.kind == kind && e.R == d.k->R && e.C == d.k->C && e.NT == d.k->NT &&
-                    e.variant == d.k->variant && e.rl == d.k->rl) d.kc = &e;
+                if (!d.kcb && e.mode == MODE_C2R_IN && e.kind == kind && e.R == d.k->R && e.C <= max_c) d.kcb = &e;
+        }
         if (p > 0) {
             d.has_tw = 1;
             d.log2Rprev = f[p - 1];
@@ -604,6 +627,7 @@ int32_t build_plan(size_t n, int device, Plan<T>** out) {
         d.k = pick_row_batch_kernel<T>(1 << ln, d.k);            // alt_row is only ever used for batches
         d.kb = d.k;
         d.kr = find_row_bulk<T>(d.kb);
+        find_real_modes(d);
         if (d.k) {
             d.tw_stage_off = off; off += (size_t(1) << ln) * sizeof(cx<T>);
             off = (off + 255) & ~size_t(255);
@@ -712,6 +736,11 @@ int32_t build_plan(size_t n, int device, Plan<T>** out) {
         CUDA_TRY(cudaFuncSetAttribute(pl->alt_row.k->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->alt_row.k->smem));
     if (pl->alt_row.kr)
         CUDA_TRY(cudaFuncSetAttribute(pl->alt_row.kr->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->alt_row.kr->smem));
+    for (const PassDesc<T>& d : {std::cref(pl->pass[0]), std::cref(pl->alt_row)}) {      // builds for batched real transforms
+        const KernelEntry<T>* real_builds[4] = {d.kc, d.kcb, d.kf, d.kfb};
+        for (const KernelEntry<T>* e : real_builds)
+            if (e) CUDA_TRY(cudaFuncSetAttribute(e->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->smem));
+    }
     if (pl->cl) {
         // usable only if the device can co-schedule at least one cluster of this shape
         cudaError_t ce = cudaFuncSetAttribute(pl->cl->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->cl->smem);
@@ -853,11 +882,37 @@ struct Io {
     long long in_bstride, out_bstride;
     int in_il, out_il;   // 0 planar, 1 interleaved, 2 interleaved with re/im swapped
     // c2r: in_re / in_im are the half-spectrum's N/2 + 1 bins and the first pass builds its input from them while loading
-    // (PassDesc::kc); pre_log2half = log2(N/2), 0 = off
+    // (PassDesc::kc / kcb); pre_log2half = log2(N/2), 0 = off
     Tw2 pre_tw2 = {nullptr, nullptr, 0};
     int pre_log2half = 0;
-    const double2* pre_wc = nullptr;     // host: W_(2 R1)^i, i < 32 (PlanR2c::pre_wc)
+    // batched r2c: the one-CTA kernel untangles its result on store (PassDesc::kf / kfb; W_N in pre_tw2).  Only the one-CTA
+    // path of run_c2c takes it (r2c_batch_dev decides).
+    int r2c_out = 0;
 };
+
+// W_(2 R1)^i, i < R1: the per-launch factors of the c2r pre-processing on load (PassParams::pre_wc), R1 = the kernel's first radix
+inline const double2* c2r_pre_wc(int r1) {
+    static const std::vector<std::vector<double2>> tabs = [] {
+        std::vector<std::vector<double2>> t(6);
+        for (int l = 0; l < 6; ++l) {
+            t[l].assign(32, make_double2(0.0, 0.0));
+            for (uint64_t i = 0; i < (1u << l); ++i) root_of_unity(i, 2u << l, t[l][i].x, t[l][i].y);
+        }
+        return t;
+    }();
+    return (r1 >= 1 && r1 <= 32 && is_pow2((size_t)r1)) ? tabs[ilog2((size_t)r1)].data() : nullptr;
+}
+
+template <typename T>
+bool many_transforms(const Plan<T>& pl, const PassDesc<T>& d, size_t batch) {
+    return d.kb != nullptr && batch > 1 && (batch << pl.log2n) >= (size_t(1) << 21);
+}
+// The MODE_R2C_OUT kernel a one-CTA pass launches for `batch` transforms (NULL: none), and whether that is kb's build.
+template <typename T>
+const KernelEntry<T>* r2c_out_kernel(const Plan<T>& pl, const PassDesc<T>& d, size_t batch, bool& many) {
+    many = many_transforms(pl, d, batch) && d.kfb != nullptr;
+    return many ? d.kfb : d.kf;
+}
 
 // k1_lo / k1_cnt (multi-pass plans, batch == 1): restrict a pass AFTER the first to the sub-transforms
 // whose first-pass output digit k1 lies in [k1_lo, k1_lo + k1_cnt) -- the unit of L2 blocking.
@@ -930,7 +985,8 @@ template <typename T>
 int32_t prepare_pass_desc(const Plan<T>& pl, const PassDesc<T>& d, int p, const PassParams<T>& base, size_t batch, long long k1_lo,
                           long long k1_cnt, PassParams<T>& prm_out, const KernelEntry<T>*& k_out, unsigned long long& blocks_out,
                           bool use_kt) {
-    const bool many = !use_kt && d.kb != nullptr && batch > 1 && (batch << pl.log2n) >= (size_t(1) << 21);
+    bool many = !use_kt && many_transforms(pl, d, batch);
+    const KernelEntry<T>* k_r2c = base.r2c_out ? r2c_out_kernel(pl, d, batch, many) : nullptr;
     const KernelEntry<T>* k = use_kt ? d.kt : many ? d.kb : d.k;
     // one-CTA batch kernel with bulk tile input / output: planar arrays, transforms back to back, 16-byte-aligned planes
     if (many && d.kr && k == d.kb && base.in_interleaved == 0 && base.out_interleaved == 0 && base.in_bstride == (long long)pl.n &&
@@ -939,10 +995,20 @@ int32_t prepare_pass_desc(const Plan<T>& pl, const PassDesc<T>& d, int p, const 
           reinterpret_cast<uintptr_t>(base.out_im)) & 15) == 0)
         k = d.kr;
     if (base.pre_log2half) {
-        if (p != 0 || use_kt || many || !d.kc) return fail(PHASTFT_ERR_INVALID_ARG, "c2r pre-processing on load: lone first pass with a MODE_C2R_IN kernel only");
-        k = d.kc;
+        const KernelEntry<T>* kc = many ? d.kcb : d.kc;
+        if (!kc && k->kind == KIND_COL) kc = d.kcb;    // a first COL pass reads no table that depends on its tile
+        if (p > 0 || use_kt || !kc) return fail(PHASTFT_ERR_INVALID_ARG, "c2r pre-processing on load: first pass or one-CTA kernel with a MODE_C2R_IN build only");
+        k = kc;
+    } else if (base.r2c_out) {
+        if (use_kt || !k_r2c) return fail(PHASTFT_ERR_INVALID_ARG, "r2c untangle on store: one-CTA kernel with a MODE_R2C_OUT build only");
+        k = k_r2c;
     }
     PassParams<T> prm = base;
+    if (base.pre_log2half) {
+        const double2* wc = c2r_pre_wc(k->first_radix);
+        if (!wc) return fail(PHASTFT_ERR_INVALID_ARG, "c2r pre-processing on load: first radix > 32");
+        memcpy(prm.pre_wc, wc, sizeof(prm.pre_wc));
+    }
     prm.batch = (int)batch;
     prm.log2A = d.log2A; prm.log2B = d.log2B; prm.log2R1 = d.log2R1; prm.log2Rprev = d.log2Rprev;
     prm.has_tw = d.has_tw; prm.tw_shift = d.tw_shift;
@@ -1020,8 +1086,10 @@ int32_t grow_workspace(const Plan<T>& pl, size_t transforms, cudaStream_t stream
     return PHASTFT_OK;
 }
 
+// `pipe`: calls may take the pipelined launch (a ring of transforms); false sizes the workspace for the chunked path, which
+// batched c2r (no pre-processing build of the pipelined pair) always takes
 template <typename T>
-int32_t plan_reserve(const Plan<T>* pl, size_t batch) {
+int32_t plan_reserve(const Plan<T>* pl, size_t batch, bool pipe = true) {
     if (!pl) return fail(PHASTFT_ERR_INVALID_ARG, "plan == NULL");
     if (pl->num_passes < 2 || batch <= 1) return PHASTFT_OK;       // one-CTA plans have no workspace
     DeviceGuard g(pl->device);
@@ -1029,7 +1097,7 @@ int32_t plan_reserve(const Plan<T>* pl, size_t batch) {
     const size_t bytes_per = pl->n * 2 * sizeof(T);
     size_t chunk = std::max<size_t>(1, l2_chunk_bytes() / bytes_per);
     chunk = std::min(chunk, batch);
-    if (pl->pipe_b && (batch << pl->log2n) >= (size_t(1) << 21)) chunk = pipe_ring_transforms(*pl, batch);
+    if (pipe && pl->pipe_b && (batch << pl->log2n) >= (size_t(1) << 21)) chunk = pipe_ring_transforms(*pl, batch);
     return grow_workspace(*pl, chunk, nullptr);
 }
 
@@ -1061,6 +1129,7 @@ int32_t run_c2c(const Plan<T>& pl, const Io<T>& io, size_t batch, T scale, cudaS
             prm.in_bstride = io.in_bstride; prm.out_bstride = io.out_bstride;
             prm.in_interleaved = io.in_il; prm.out_interleaved = io.out_il;
             prm.scale = scale;
+            prm.pre_tw2 = io.pre_tw2; prm.pre_log2half = io.pre_log2half; prm.r2c_out = io.r2c_out;
             if (pass_events && done == 0) CUDA_TRY(cudaEventRecord(pass_events[0], stream));
             int32_t st = launch_pass(pl, which, prm, nb, stream);
             if (st) return st;
@@ -1072,8 +1141,10 @@ int32_t run_c2c(const Plan<T>& pl, const Io<T>& io, size_t batch, T scale, cudaS
         }
         return PHASTFT_OK;
     }
+    if (io.r2c_out) return fail(PHASTFT_ERR_INVALID_ARG, "r2c untangle on store: one-CTA plans only");
     // ---- both passes in one cluster launch: no workspace, HBM sees the batch once in and once out ----------------
-    if (pl.cl && batch >= pl.cl_min_batch) {
+    // (its first pass has no c2r pre-processing build)
+    if (pl.cl && batch >= pl.cl_min_batch && !io.pre_log2half) {
         const size_t max_chunk = (size_t(1) << 30) / (size_t)pl.cl->K;        // grid = transforms x K CTAs
         for (size_t done = 0; done < batch; done += max_chunk) {
             const size_t nb = std::min(batch - done, max_chunk);
@@ -1120,7 +1191,9 @@ int32_t run_c2c(const Plan<T>& pl, const Io<T>& io, size_t batch, T scale, cudaS
     // pipelined two-pass launch (see fft_pipe2_kernel): the workspace is a ring of transforms instead of the whole chunk
     const PipeEntry<T>* pipe = nullptr;
     if (pl.num_passes == 2 && !pass_events) {
-        if (batch > 1 && (batch << pl.log2n) >= (size_t(1) << 21)) pipe = pl.pipe_b;
+        // (no c2r pre-processing build of its passes; its TMA tile input reads planar data only)
+        if (batch > 1 && (batch << pl.log2n) >= (size_t(1) << 21) && !io.pre_log2half && !(pl.pipe_b && pl.pipe_b->mode == 1 && io.in_il != 0))
+            pipe = pl.pipe_b;
         else if (batch == 1 && io.in_il == 0 && io.out_il == 0 && !io.pre_log2half) pipe = pl.pipe_1;
     }
     size_t ws_need = chunk;
@@ -1221,7 +1294,6 @@ int32_t run_c2c(const Plan<T>& pl, const Io<T>& io, size_t batch, T scale, cudaS
             prm.in_im = io.in_im ? io.in_im + b * io.in_bstride : nullptr;
             prm.in_bstride = io.in_bstride; prm.in_interleaved = io.in_il;
             prm.pre_tw2 = io.pre_tw2; prm.pre_log2half = io.pre_log2half;
-                if (io.pre_wc) memcpy(prm.pre_wc, io.pre_wc, sizeof(prm.pre_wc));
             prm.out_re = pl.ws_re; prm.out_im = pl.ws_im; prm.out_bstride = (long long)pl.n;
             if (pass_events && b == 0) CUDA_TRY(cudaEventRecord(pass_events[0], stream));
             int32_t st = launch_pass(pl, 0, prm, 1, stream);
@@ -1272,7 +1344,6 @@ int32_t run_c2c(const Plan<T>& pl, const Io<T>& io, size_t batch, T scale, cudaS
                 prm.in_bstride = io.in_bstride;
                 prm.in_interleaved = io.in_il;
                 prm.pre_tw2 = io.pre_tw2; prm.pre_log2half = io.pre_log2half;
-                if (io.pre_wc) memcpy(prm.pre_wc, io.pre_wc, sizeof(prm.pre_wc));
             } else {
                 prm.in_re = pl.ws_re; prm.in_im = pl.ws_im; prm.in_bstride = (long long)pl.n;
                 prm.in_interleaved = il;
@@ -1732,7 +1803,6 @@ struct PlanR2c {
     unsigned char* tw_dev = nullptr;   // two-level W_n table for the untangle / preprocess twiddles
     size_t hi_elems = 0, lo_elems = 0;
     int lo_bits = 0;
-    double2 pre_wc[32];                // W_(2 R1)^i for the fused c2r first pass (R1 = first radix of inner->pass[0].kc)
     mutable std::mutex mu;
     mutable std::mutex host_mu;        // held for a whole *_host call (lock order: host_mu, then mu)
     mutable T* d_real = nullptr;       // host-API staging: N reals
@@ -1772,11 +1842,6 @@ int32_t build_plan_r2c(size_t n, int device, PlanR2c<T>** out) {
     for (size_t l = 0; l < pl->lo_elems; ++l) root_of_unity(l, n, tab[pl->hi_elems + l].x, tab[pl->hi_elems + l].y);
     CUDA_TRY(cudaMalloc(&pl->tw_dev, tab.size() * sizeof(double2)));
     CUDA_TRY(cudaMemcpy(pl->tw_dev, tab.data(), tab.size() * sizeof(double2), cudaMemcpyHostToDevice));
-    memset(pl->pre_wc, 0, sizeof(pl->pre_wc));
-    if (pl->inner->num_passes >= 2 && pl->inner->pass[0].kc) {
-        const uint64_t r1 = (uint64_t)pl->inner->pass[0].kc->first_radix;
-        for (uint64_t i = 0; i < r1 && i < 32; ++i) root_of_unity(i, 2 * r1, pl->pre_wc[i].x, pl->pre_wc[i].y);
-    }
     // c2r scratch for the allocating variants lives in the plan (r2c.rs:716-718 allocates per call)
     CUDA_TRY(cudaMalloc(&pl->d_scr_re, (n / 2) * sizeof(T)));
     CUDA_TRY(cudaMalloc(&pl->d_scr_im, (n / 2) * sizeof(T)));
@@ -1838,7 +1903,7 @@ int32_t c2r_dev(const PlanR2c<T>* pl, const T* d_ire, const T* d_iim, T* d_out, 
     if (fuse_env && fuse_size && in.num_passes >= 2 && in.pass[0].kc && !(in.cl && in.cl_min_batch <= 1) && !in.pipe_1) {
         Io<T> io;
         io.in_re = d_ire; io.in_im = d_iim; io.in_il = 0; io.in_bstride = (long long)half;
-        io.pre_tw2 = r2c_tw2(pl); io.pre_log2half = ilog2(half); io.pre_wc = pl->pre_wc;
+        io.pre_tw2 = r2c_tw2(pl); io.pre_log2half = ilog2(half);
         io.out_re = d_out; io.out_im = nullptr; io.out_il = 2; io.out_bstride = (long long)half;
         return run_c2c(in, io, 1, T(1) / (T)half, stream);
     }
@@ -1875,6 +1940,84 @@ int32_t c2r_dev(const PlanR2c<T>* pl, const T* d_ire, const T* d_iim, T* d_out, 
         pl->scr_used = true;
     }
     return st;
+}
+
+// Batched device-resident r2c / c2r (strides in elements of T).  The real side is read or written as complex pairs, so its
+// stride must be even and its base aligned to 2 * sizeof(T).  Checked before anything is launched.
+template <typename T>
+int32_t check_real_batch(const PlanR2c<T>* pl, const void* p0, const void* p1, const void* p2, const T* real, size_t real_stride,
+                         size_t spec_stride, size_t batch) {
+    if (!pl || !p0 || !p1 || !p2) return fail(PHASTFT_ERR_INVALID_ARG, "NULL argument");
+    const size_t n = pl->n, half = n / 2;
+    if (real_stride < n) return fail(PHASTFT_ERR_INVALID_ARG, "real-side stride < N");
+    if (spec_stride < half + 1) return fail(PHASTFT_ERR_INVALID_ARG, "spectrum stride < N/2 + 1");
+    if (real_stride & 1) return fail(PHASTFT_ERR_INVALID_ARG, "real-side stride must be even (the reals are read as complex pairs)");
+    if (reinterpret_cast<uintptr_t>(real) % (2 * sizeof(T))) return fail(PHASTFT_ERR_INVALID_ARG, "real-side base not aligned to 2 * sizeof(T)");
+    const size_t lim = (size_t(1) << 62) / sizeof(T);
+    if (batch > 1 && (batch - 1) > (lim - n) / std::max(real_stride, spec_stride)) return fail(PHASTFT_ERR_INVALID_ARG, "batch * stride too large");
+    return PHASTFT_OK;
+}
+
+// r2c of the inner plan's one-CTA kernel with the untangle in its store (MODE_R2C_OUT), or NULL: the half-length c2c and the
+// separate untangle sweep.  PHASTFT_R2C_FUSE=0 forces the latter (equivalence tests, measurement).
+template <typename T>
+const KernelEntry<T>* r2c_fused_kernel(const Plan<T>& in, size_t batch) {
+    const char* e = getenv("PHASTFT_R2C_FUSE");
+    if (e && atoi(e) == 0) return nullptr;
+    const bool one_cta = in.num_passes == 1 || (in.alt_row.k && batch >= in.alt_row_min_batch);     // as run_c2c decides
+    if (!one_cta) return nullptr;
+    bool many = false;
+    return r2c_out_kernel(in, in.num_passes == 1 ? in.pass[0] : in.alt_row, batch, many);
+}
+
+template <typename T>
+int32_t r2c_batch_dev(const PlanR2c<T>* pl, const T* d_in, T* d_ore, T* d_oim, size_t batch, size_t in_stride, size_t out_stride,
+                      cudaStream_t stream) {
+    int32_t st = check_real_batch(pl, d_in, d_ore, d_oim, d_in, in_stride, out_stride, batch);
+    if (st || batch == 0) return st;
+    if (batch == 1) return r2c_dev(pl, d_in, d_ore, d_oim, stream);          // bit-identical to the single call by construction
+    DeviceGuard g(pl->device);
+    const size_t half = pl->n / 2;
+    const Plan<T>& in = *pl->inner;
+    Io<T> io;
+    io.in_re = d_in; io.in_im = nullptr; io.in_il = 1; io.in_bstride = (long long)(in_stride / 2);
+    io.out_re = d_ore; io.out_im = d_oim; io.out_il = 0; io.out_bstride = (long long)out_stride;
+    if (r2c_fused_kernel(in, batch)) {
+        io.r2c_out = 1; io.pre_tw2 = r2c_tw2(pl);
+        return run_c2c(in, io, batch, T(1), stream);
+    }
+    st = run_c2c(in, io, batch, T(1), stream);
+    if (st) return st;
+    // untangle sweep over every member: (member, pair) flattened into grid.x, launches of at most 2^30 blocks
+    RealParams<T> rp;
+    memset(&rp, 0, sizeof(rp));
+    rp.bstride = (long long)out_stride; rp.log2half = ilog2(half); rp.tw2 = r2c_tw2(pl);
+    const size_t q1 = half / 2 + 1;
+    const size_t max_members = (size_t(256) << 30) / q1;
+    for (size_t done = 0; done < batch; done += max_members) {
+        const size_t nb = std::min(max_members, batch - done);
+        rp.re = d_ore + done * out_stride; rp.im = d_oim + done * out_stride;
+        r2c_untangle_batch_kernel<T><<<(unsigned)((nb * q1 + 255) / 256), 256, 0, stream>>>(rp, (long long)nb);
+        CUDA_TRY(cudaGetLastError());
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+    }
+    return PHASTFT_OK;
+}
+
+// Every batched c2r path pre-processes on load (first pass, or the one-CTA kernel): no scratch that would grow with the batch.
+template <typename T>
+int32_t c2r_batch_dev(const PlanR2c<T>* pl, const T* d_ire, const T* d_iim, T* d_out, size_t batch, size_t in_stride, size_t out_stride,
+                      cudaStream_t stream) {
+    int32_t st = check_real_batch(pl, d_ire, d_iim, d_out, d_out, out_stride, in_stride, batch);
+    if (st || batch == 0) return st;
+    if (batch == 1) return c2r_dev<T>(pl, d_ire, d_iim, d_out, nullptr, nullptr, stream);
+    DeviceGuard g(pl->device);
+    const size_t half = pl->n / 2;
+    Io<T> io;
+    io.in_re = d_ire; io.in_im = d_iim; io.in_il = 0; io.in_bstride = (long long)in_stride;
+    io.pre_tw2 = r2c_tw2(pl); io.pre_log2half = ilog2(half);
+    io.out_re = d_out; io.out_im = nullptr; io.out_il = 2; io.out_bstride = (long long)(out_stride / 2);
+    return run_c2c(*pl->inner, io, batch, T(1) / (T)half, stream);
 }
 
 template <typename T>
@@ -2112,6 +2255,18 @@ void phastft_options_guess(size_t input_size, phastft_options* out) {
     int32_t phastft_c2r_##SFX##_dev(const phastft_plan_r2c_##SFX* p, const T* ire, const T* iim, T* out, T* sre,        \
                                     T* sim, void* s) {                                                                  \
         return c2r_dev<T>(AS_CR2C(T, p), ire, iim, out, sre, sim, (cudaStream_t)s);                                     \
+    }                                                                                                                   \
+    int32_t phastft_r2c_##SFX##_dev_batch(const phastft_plan_r2c_##SFX* p, const T* in, T* ore, T* oim, size_t batch,  \
+                                          size_t in_stride, size_t out_stride, void* s) {                               \
+        return r2c_batch_dev<T>(AS_CR2C(T, p), in, ore, oim, batch, in_stride, out_stride, (cudaStream_t)s);            \
+    }                                                                                                                   \
+    int32_t phastft_c2r_##SFX##_dev_batch(const phastft_plan_r2c_##SFX* p, const T* ire, const T* iim, T* out,         \
+                                          size_t batch, size_t in_stride, size_t out_stride, void* s) {                 \
+        return c2r_batch_dev<T>(AS_CR2C(T, p), ire, iim, out, batch, in_stride, out_stride, (cudaStream_t)s);           \
+    }                                                                                                                   \
+    int32_t phastft_plan_r2c_##SFX##_reserve(const phastft_plan_r2c_##SFX* p, size_t batch) {                           \
+        if (!p) return fail(PHASTFT_ERR_INVALID_ARG, "plan == NULL");                                                   \
+        return plan_reserve<T>(AS_CR2C(T, p)->inner, batch, false);                                                     \
     }
 
 DEFINE_DIT_API(double, f64)

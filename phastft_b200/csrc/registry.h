@@ -86,7 +86,8 @@ KernelEntry<T> make_entry_async() {
     e.smem = PK::SMEM_BYTES;
     e.fn = reinterpret_cast<const void*>(&fft_pass_async_kernel<T, RL, C, NT, KIND, MODE, VARIANT, MINB>);
     e.rl = radix_string<RL>();
-    e.radices = e.rl + (MODE == MODE_TMA_IN ? ",tma" : MODE == MODE_BULK_IN ? ",bulk" : MODE == MODE_C2R_IN ? ",c2r" : ",bulk-io");
+    e.radices = e.rl + (MODE == MODE_TMA_IN ? ",tma" : MODE == MODE_BULK_IN ? ",bulk" : MODE == MODE_C2R_IN ? ",c2r" :
+                        MODE == MODE_R2C_OUT ? ",r2c" : ",bulk-io");
     for (int q = 0; q < RL::S && q < 8; ++q) e.rads[q] = RL::rad(q);
     if (ID) e.radices += ",v" + std::to_string(ID);
     return e;
@@ -97,6 +98,18 @@ template <typename T, int KIND, int C, int NT, int VARIANT, int MINB, int ID, in
 void push_entry(std::vector<KernelEntry<T>>& v) {
     v.push_back(make_entry_v<T, KIND, C, NT, VARIANT, MINB, ID, Rs...>());
     if constexpr (KIND == KIND_COL) v.push_back(make_entry_async<T, KIND, C, NT, MODE_C2R_IN, VARIANT, MINB, ID, Rs...>());
+}
+
+// a one-CTA kernel plus the builds of the same tile for batched real transforms: c2r pre-processing on load (every tile) and
+// r2c untangle on store (tiles with a shared-memory stage to untangle from, S >= 2).  MINB_C2R / MINB_R2C: their
+// minimum-blocks bounds, the plain build's resident CTAs per SM so that they keep its occupancy (0 where that would spill)
+template <typename T, int C, int NT, int VARIANT, int MINB, int ID, int MINB_C2R, int MINB_R2C, int... Rs>
+void push_row(std::vector<KernelEntry<T>>& v) {
+    static_assert((MINB_C2R == 0 || MINB_C2R >= MINB) && (MINB_R2C == 0 || MINB_R2C >= MINB), "a real build keeps the plain build's bound");
+    v.push_back(make_entry_v<T, KIND_ROW, C, NT, VARIANT, MINB, ID, Rs...>());
+    v.push_back(make_entry_async<T, KIND_ROW, C, NT, MODE_C2R_IN, VARIANT, MINB_C2R ? MINB_C2R : MINB, ID, Rs...>());
+    if constexpr (sizeof...(Rs) >= 2)
+        v.push_back(make_entry_async<T, KIND_ROW, C, NT, MODE_R2C_OUT, VARIANT, MINB_R2C ? MINB_R2C : MINB, ID, Rs...>());
 }
 
 template <typename T, int KIND, int C, int NT, int... Rs>

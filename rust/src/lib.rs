@@ -186,6 +186,35 @@ pub unsafe fn c2r_fft_f32_device(d_in_re: *const f32, d_in_im: *const f32, d_out
     check(ffi::phastft_c2r_f32_dev(planner.raw, d_in_re, d_in_im, d_output, d_scratch_re, d_scratch_im, stream));
 }
 
+/// Batched device-resident real transforms (`phastft_{r2c,c2r}_*_dev_batch`): member `b` of the real side at
+/// `b * real_stride`, of the spectrum at `b * spectrum_stride` (elements).  Panics with code 13 on a bad stride or alignment.
+///
+/// # Safety
+/// Device pointers on the planner's device, `batch` members long at the given strides; the real-side stride even and its
+/// base aligned to two elements.
+pub unsafe fn r2c_fft_f64_device_batch(d_input: *const f64, d_out_re: *mut f64, d_out_im: *mut f64, planner: &PlannerR2c64, batch: usize,
+                                       in_stride: usize, out_stride: usize, stream: *mut std::os::raw::c_void) {
+    check(ffi::phastft_r2c_f64_dev_batch(planner.raw, d_input, d_out_re, d_out_im, batch, in_stride, out_stride, stream));
+}
+/// # Safety
+/// As [`r2c_fft_f64_device_batch`].
+pub unsafe fn c2r_fft_f64_device_batch(d_in_re: *const f64, d_in_im: *const f64, d_output: *mut f64, planner: &PlannerR2c64, batch: usize,
+                                       in_stride: usize, out_stride: usize, stream: *mut std::os::raw::c_void) {
+    check(ffi::phastft_c2r_f64_dev_batch(planner.raw, d_in_re, d_in_im, d_output, batch, in_stride, out_stride, stream));
+}
+/// # Safety
+/// As [`r2c_fft_f64_device_batch`].
+pub unsafe fn r2c_fft_f32_device_batch(d_input: *const f32, d_out_re: *mut f32, d_out_im: *mut f32, planner: &PlannerR2c32, batch: usize,
+                                       in_stride: usize, out_stride: usize, stream: *mut std::os::raw::c_void) {
+    check(ffi::phastft_r2c_f32_dev_batch(planner.raw, d_input, d_out_re, d_out_im, batch, in_stride, out_stride, stream));
+}
+/// # Safety
+/// As [`r2c_fft_f64_device_batch`].
+pub unsafe fn c2r_fft_f32_device_batch(d_in_re: *const f32, d_in_im: *const f32, d_output: *mut f32, planner: &PlannerR2c32, batch: usize,
+                                       in_stride: usize, out_stride: usize, stream: *mut std::os::raw::c_void) {
+    check(ffi::phastft_c2r_f32_dev_batch(planner.raw, d_in_re, d_in_im, d_output, batch, in_stride, out_stride, stream));
+}
+
 // ------------------------------------------------------------------------------------------------
 // r2c / c2r  (algorithms/r2c.rs:521-895)
 // ------------------------------------------------------------------------------------------------

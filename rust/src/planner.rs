@@ -67,7 +67,7 @@ impl_planner_dit!(PlannerDit32, ffi::phastft_plan_dit_f32, phastft_plan_dit_f32_
                   phastft_plan_dit_f32_size, phastft_plan_dit_f32_describe, phastft_plan_dit_f32_reserve);
 
 macro_rules! impl_planner_r2c {
-    ($name:ident, $raw:ty, $create:ident, $destroy:ident) => {
+    ($name:ident, $raw:ty, $create:ident, $destroy:ident, $reserve:ident) => {
         pub struct $name {
             pub(crate) raw: *mut $raw,
         }
@@ -80,6 +80,10 @@ macro_rules! impl_planner_r2c {
                 check(unsafe { ffi::$create(n, device(), &mut raw) });
                 Self { raw }
             }
+            /// Additive: size the half-length transform's workspace for batched calls of up to `batch` members now.
+            pub fn reserve(&self, batch: usize) {
+                check(unsafe { ffi::$reserve(self.raw, batch) });
+            }
         }
         impl Drop for $name {
             fn drop(&mut self) {
@@ -88,5 +92,7 @@ macro_rules! impl_planner_r2c {
         }
     };
 }
-impl_planner_r2c!(PlannerR2c64, ffi::phastft_plan_r2c_f64, phastft_plan_r2c_f64_create, phastft_plan_r2c_f64_destroy);
-impl_planner_r2c!(PlannerR2c32, ffi::phastft_plan_r2c_f32, phastft_plan_r2c_f32_create, phastft_plan_r2c_f32_destroy);
+impl_planner_r2c!(PlannerR2c64, ffi::phastft_plan_r2c_f64, phastft_plan_r2c_f64_create, phastft_plan_r2c_f64_destroy,
+                  phastft_plan_r2c_f64_reserve);
+impl_planner_r2c!(PlannerR2c32, ffi::phastft_plan_r2c_f32, phastft_plan_r2c_f32_create, phastft_plan_r2c_f32_destroy,
+                  phastft_plan_r2c_f32_reserve);
